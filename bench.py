@@ -1,6 +1,6 @@
 """bench.py - frame-pairs/sec of the adversarial train step at 256x448 (BASELINE.json metric) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload train|gen_fwd|ensemble]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload train|gen_fwd|ensemble] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Headline workload `train` (BASELINE.json configs[1]/[2]): DAVIS2016-shaped adversarial training, 4 frame pairs per GPU, PWC-Net at
@@ -13,6 +13,9 @@ Other arms (not the headline; BASELINE.json configs[0] and configs[4]):
   --workload ensemble   multi-crop ensemble inference (test_generator_ensemble.py / generate_buffer_DAVIS2016.sh): per frame pair the
                         four central crops -> PWC-Net 384x640 -> generator at the default 192x384; frames sharded over the ranks
 `--impl reference` times the CPU restatement of the same graph (oracle/; TF 1.13 cannot be installed here) on the host cores.
+`--dump-outputs DIR` writes what the last timed step returned to its caller as DIR/<name>.npy (train: losses, masks, flows, trained
+weights; gen_fwd / ensemble: masks), rank 0's share under data parallelism: inputs and weights are seeded, so two builds run with the
+same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -22,6 +25,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -31,6 +35,7 @@ METRIC = 'frame-pairs/sec adversarial train step 256x448'
 H, W, BPG = 256, 448, 4
 WORKLOAD_TRAIN = 'DAVIS2016-shaped adversarial train 256x448, batch 4/GPU, PWC-Net 384x640 in loop, 1 rec : 3 gen (configs[1])'
 GFLOP_PER_PAIR_STEP = 228.1    # SURVEY.md section 8(d): algorithmic conv FLOPs of one frame pair through one step, 1R:3G cycle average
+DUMP_LIMIT = 64 << 20          # bytes of all --dump-outputs arrays together
 
 
 def peaks():
@@ -110,6 +115,13 @@ def cpu_reference(steps, warmup, batch=1, threads=None):
     return batch * len(times) / tot, threads, tot / len(times) * 1e3, ''.join(kinds)
 
 
+def reference_steps(args, most):
+    """The CPU arm takes seconds per step, so it times at most `most` steps; it says so on stderr when --steps asks for more."""
+    if args.steps > most:
+        print('bench.py: the reference arm times %d steps, not the %d asked for' % (most, args.steps), file=sys.stderr)
+    return min(args.steps, most)
+
+
 def run_reference(args):
     rank = int(os.environ.get('RANK', '0'))
     if rank != 0:
@@ -117,7 +129,7 @@ def run_reference(args):
     if args.workload != 'train':
         return run_reference_other(args)
     # same config as our arm at N = 1 (4 frame pairs per step, same 1R:3G schedule); bounded to <= 12 timed steps = three cycles
-    steps, warmup = max(1, min(args.steps, 12)), min(max(args.warmup, 1), 1)
+    steps, warmup = reference_steps(args, 12), min(max(args.warmup, 1), 1)
     v, threads, ms, kinds = cpu_reference(steps, warmup, batch=BPG)
     line = {'impl': 'reference', 'metric': METRIC, 'value': v, 'unit': 'frame-pairs/s', 'n_gpus': args.gpus, 'steps': steps, 'warmup': warmup,
             'ms_per_step': ms, 'higher_is_better': True, 'scaling': 'weak', 'vs_baseline': None, 'dtype': 'f32', 'data': 'synthetic',
@@ -196,6 +208,34 @@ def dominant_launch_roofline(graph, reps=20):
     return fl, med, desc
 
 
+def train_outputs(L):
+    """What the last train step handed its caller, copied to the host: the four loss scalars (summed over the ranks, as
+    AdversarialLearner.step reports them), this rank's masks, recovered flows and generator input flow, and the weights of both
+    trained networks, each flattened in variable-name order.  Every rank must call it: the loss read is a collective under data
+    parallelism.  The copies matter: any later step overwrites the graph's buffers in place."""
+    g = L.graph
+    g.pipeline_drain()
+    torch.cuda.synchronize()
+    ls = g.losses(reduce=L._allreduce())
+    out = {'losses': torch.tensor([ls[k] for k in ('generator', 'recover', 'red_rate', 'red_rate_compl')], dtype=torch.float64),
+           'masks': g.mask.cpu(), 'recovered_flows': g.pred.cpu(), 'flow': g.flow.cpu()}
+    params = g.export_params()
+    for net in ('MaskNet', 'FlownetS'):
+        out['weights_' + net] = torch.cat([params[k].reshape(-1) for k in sorted(params) if k.startswith(net + '/')]).cpu()
+    return out
+
+
+def dump_outputs(out_dir, arrays):
+    """arrays: name -> tensor, written as out_dir/<name>.npy in float64 (if it is float64) or float32."""
+    arrays = {k: v.detach().to('cpu', torch.float64 if v.dtype == torch.float64 else torch.float32).numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise ValueError('--dump-outputs: %d bytes exceed the %d-byte limit' % (total, DUMP_LIMIT))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + '.npy'), a)
+
+
 def run_ours(args):
     import torch.distributed as dist
     from unsupervised_detection_b200.common_flags import Config
@@ -252,6 +292,7 @@ def run_ours(args):
     ms_e2e = timed(lambda i: L.step(pool[(i + off) % 2], fetch_losses=True, next_batch=pool[(i + off + 1) % 2]), K)
     smp.stop_flag = True
     smp.join(timeout=2)
+    outputs = train_outputs(L) if args.dump_outputs else None     # copied before the per-kind timings below train further
     # each step kind on its own (SURVEY 8d asks for the 1R:3G cycle average AND the two kinds separately); single GPU only, after the
     # headline measurements, and never allowed to take them down
     by_kind = None
@@ -270,6 +311,8 @@ def run_ours(args):
     launches = sum(g.launches_per_step('R' if (i % 4) == 3 else 'G') for i in range(K))
     if rank != 0:
         return
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     pk, src = peaks()
     fl, ms_conv, nconv = conv_roofline(g)
     ach = fl / (ms_conv * 1e-3) / 1e12
@@ -391,6 +434,8 @@ def run_ours_other(args):
         ms_dev, ms_e2e = float(t[0]), float(t[1])
         if rank != 0:
             return
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {'masks': mask_host})      # the mask the last timed step read back for its caller
         gflop = 8.437                                        # SURVEY App. B.1 at 128x224
         cv = cores = None
         if not args.no_cpu:
@@ -440,6 +485,8 @@ def run_ours_other(args):
     ms_dev, ms_e2e = float(t[0]), float(t[1])
     if rank != 0:
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {'masks': g.mask})              # the last timed inference's pred_masks, one row per crop
     ncrop = len(L.test_crops)
     gflop = ncrop * 123.8                                    # SURVEY 8(d): PWC-Net + generator @192x384 per crop
     cv = cores = None
@@ -505,11 +552,11 @@ def cpu_ensemble(frames):
 
 def run_reference_other(args):
     if args.workload == 'gen_fwd':
-        steps = max(1, min(args.steps, 20))
+        steps = reference_steps(args, 20)
         v, th = cpu_gen_fwd(steps)
         metric, wl = 'frame-pairs/sec mask-net forward 128x224 (BASELINE configs[0])', 'test_generator.py single frame pair 128x224, precomputed flow, mask-net forward only (configs[0])'
     else:
-        steps = max(1, min(args.steps, 3))
+        steps = reference_steps(args, 3)
         v, th = cpu_ensemble(steps)
         metric, wl = 'frame-pairs/sec multi-crop ensemble inference 192x384 (BASELINE configs[4])', 'generate_buffer ensemble inference: 4 central crops per frame pair, PWC-Net 384x640 + generator 192x384 (configs[4])'
     print(json.dumps({'impl': 'reference', 'metric': metric, 'value': v, 'unit': 'frame-pairs/s', 'n_gpus': args.gpus, 'steps': steps, 'warmup': 1,
@@ -528,7 +575,12 @@ def main():
     ap.add_argument('--no-cpu', action='store_true', help='skip the cpu_baseline leg')
     ap.add_argument('--workload', default='train', choices=['train', 'gen_fwd', 'ensemble'],
                     help='train = the headline metric; gen_fwd = BASELINE configs[0]; ensemble = BASELINE configs[4]')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the outputs of the last timed step as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs needs --impl ours')
     if args.impl == 'reference':
         run_reference(args)
     else:
