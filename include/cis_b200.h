@@ -102,6 +102,11 @@ typedef struct {
     int32_t OH, OW, oa, ob;   /* output extent and offset inside the (DH, DW) destination grid (stride osh / osw) */
     const void* wpack;        /* pre-tiled weights of this sub-problem */
   } sub[4];
+  /* Compact thin halo (halo = 1, all sources together <= 16 channels): the halo is staged as 8-channel planes of 16 B per pixel
+   * ([plane][Hh][Wh][8], SWIZZLE_NONE) and every "tap" of dh / dw / ntaps / ph_tap / sub[] is one K=16 MMA: for 8-channel inputs two
+   * x-adjacent taps (the second K half is the next pixel), for 16 channels one tap (the second K half is the next plane).  wpack then
+   * holds one BN x 32 B no-swizzle tile per MMA (cis_pack_weights_tiled, layout 1). */
+  int32_t thin;
 } CisConv;
 
 /* Weight gradient of the same convolution: dWp[co][(t,c)] = sum_rows g[row][co] * A[row][(t,c)]  (fp32).  The reduction over rows
@@ -151,9 +156,10 @@ int cis_conv_wgrad(const CisWgrad* d, cis_stream_t stream);
 int cis_pack_weights(const float* w, const int32_t* kmap, int32_t K_pad, int32_t rows, int32_t cout, int32_t sn, const int32_t* nmap,
                      void* wp, cis_stream_t stream);
 /* halo-kernel operand: out[(ny, chunk, tap)][n][64] bf16 blocks of BN x 128 B with the SWIZZLE_128B pattern pre-applied; kmap is the
- * same tap-major map (k = tap*cin8 + channel). */
+ * same tap-major map (k = tap*cin8 + channel).  layout 1 (compact thin halo, CisConv.thin): cin8 = 16, one BN x 32 B no-swizzle
+ * block [K half][n][8] per MMA ("tap"). */
 int cis_pack_weights_tiled(const float* w, const int32_t* kmap, int32_t cin8, int32_t ntaps, int32_t n_tiles, int32_t BN, int32_t cout,
-                           int32_t sn, const int32_t* nmap, void* out, cis_stream_t stream);
+                           int32_t sn, const int32_t* nmap, void* out, int32_t layout, cis_stream_t stream);
 /* dw[kmap[k] + n] = sum_{s < nsplit} dwp[s](n, k) for kmap[k] >= 0, n < cout (fixed summation order; forward orientation, sn = 1);
  * and, when colpart != NULL, the bias gradient db[c] = sum_{b < nblocks} colpart[b][c], c < nch (the partials of cis_colsum).
  * layout = how cis_conv_wgrad stored a slice: 0 = [cout][K_pad] (CisWgrad.tma == 2), 1 = float4 columns [K_pad/4][cout][4] (tma 0 / 1). */

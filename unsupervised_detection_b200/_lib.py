@@ -47,7 +47,7 @@ class CisConv(C.Structure):
                 ('ey', C.c_int32), ('ex', C.c_int32),
                 ('splits', C.c_int32), ('sk_scratch', C.c_void_p), ('sk_counters', C.c_void_p),
                 ('nph', C.c_int32), ('ph_tap', C.c_int32 * 5), ('sk_cluster', C.c_int32),
-                ('nsub', C.c_int32), ('sub', CisSub * 4)]
+                ('nsub', C.c_int32), ('sub', CisSub * 4), ('thin', C.c_int32)]
 
 
 class CisWgrad(C.Structure):
@@ -66,7 +66,7 @@ _PROTOS = {
     'cis_conv_igemm': [C.POINTER(CisConv)],
     'cis_conv_wgrad': [C.POINTER(CisWgrad)],
     'cis_pack_weights': [_p, _p, _i32, _i32, _i32, _i32, _p, _p],
-    'cis_pack_weights_tiled': [_p, _p, _i32, _i32, _i32, _i32, _i32, _i32, _p, _p],
+    'cis_pack_weights_tiled': [_p, _p, _i32, _i32, _i32, _i32, _i32, _i32, _p, _p, _i32],
     'cis_unpack_wgrad': [_p, _p, _i32, _i32, _i32, _p, _p, _i32, _i32, _p, _i32],
     'cis_bn_fold': [_p, _p, _p, _p, _i64, _i32, _p, _p],
     'cis_param_multi': [_p, _i32, _i32],

@@ -587,6 +587,8 @@ __global__ void __launch_bounds__(kGThreads) conv_igemm_kernel(const __grid_cons
 // non-1024 SBO are legal with base_offset = 0.  im2col traffic drops from k*k x to ~1.3 x and the packed weights of a
 // (tap, chunk) are reused by the MT tiles.
 static constexpr int kHaloMaxBStages = 8;
+// compact thin halo: bytes between the 8-channel planes of one halo stage (16 B per pixel, 128-byte aligned planes)
+__host__ __device__ __forceinline__ uint32_t thin_plane_bytes(int HP) { return ((uint32_t)HP * 16u + 127u) & ~127u; }
 struct HaloMaps {
   // one 4-D (C, W, H, N) SWIZZLE_128B map per (concat source, stride-2 phase): index si * nph + phase; box = (64, Wh, Hh, 1)
   CUtensorMap m[CIS_MAX_SRC * 4];
@@ -648,8 +650,7 @@ __device__ __forceinline__ void halo_issue_mt1(const uint32_t tmem, const uint32
 template <int NK>
 __device__ __forceinline__ void halo_issue_stage(const uint32_t tmem, const uint32_t hlo, uint32_t blo, const uint32_t* s_aoff, const int gt,
                                                  const int MT, const int BN, const uint32_t ahi, const uint32_t bhi, const uint32_t a_mstep,
-                                                 const uint32_t idesc, const bool first) {
-  const uint32_t bstep = (uint32_t)(BN * 128) >> 4;
+                                                 const uint32_t bstep, const uint32_t idesc, const bool first) {
   if (NK == 1 && MT == 1) {      // single-MMA taps: the loop overhead below would dominate
     halo_issue_mt1<NK>(tmem, hlo, blo, s_aoff, gt, bstep, ahi, bhi, idesc, first);
     return;
@@ -682,7 +683,9 @@ __global__ void __launch_bounds__(HaloCfg<BN>::kThreads, HaloCfg<BN>::kMinCtas) 
   // bulk copy): the single MMA-issuing thread then pays the per-stage cost (mbarrier wait, tcgen05 fence, election, commits: several
   // hundred clocks of dependent single-thread latency, measured with the CIS_TRACE build) once per 4*MT*G MMAs instead of once per
   // 4*MT -- that cost, not the tensor pipe, bounded every launch of round 1.
-  constexpr int kBStage = BN * 128;
+  // Compact thin halo (p.thin): 8-channel planes of 16 B per pixel, one K=16 MMA per "tap" entry, BN x 32 B weight tiles.
+  const int thin = p.thin;
+  const int kBStage = thin ? BN * 32 : BN * 128;
   constexpr int kHMmaWarp_ = HaloCfg<BN>::kMmaWarp, kHThreads_ = HaloCfg<BN>::kThreads;
   extern __shared__ uint8_t smem_raw[];
   __shared__ uint64_t bars[2 * 2 + 2 * kHaloMaxBStages + 1];
@@ -732,7 +735,7 @@ __global__ void __launch_bounds__(HaloCfg<BN>::kThreads, HaloCfg<BN>::kMinCtas) 
   pdl_launch_dependents();
   const uint32_t ncols = (MT * BN <= 32) ? 32u : (MT * BN <= 64) ? 64u : (MT * BN <= 128) ? 128u : (MT * BN <= 256) ? 256u : 512u;
 
-  if (tid < ntaps) s_aoff[tid] = (uint32_t)((p.dh[tap0 + tid] * Wh + p.dw[tap0 + tid]) * 8);   // * 128 B / 16
+  if (tid < ntaps) s_aoff[tid] = (uint32_t)((p.dh[tap0 + tid] * Wh + p.dw[tap0 + tid]) * (thin ? 1 : 8));   // * pixel bytes / 16
   if (tid < p.nsrc) {
     s_src[tid].ptr = reinterpret_cast<const __nv_bfloat16*>(p.src[tid].ptr);
     s_src[tid].pitch = p.src[tid].pitch;
@@ -790,6 +793,18 @@ __global__ void __launch_bounds__(HaloCfg<BN>::kThreads, HaloCfg<BN>::kMinCtas) 
           while (si < p.nsrc - 1 && c >= s_src[si].chunks) {
             c -= s_src[si].chunks;
             ++si;
+          }
+          if (thin) {
+            // one 16-byte-per-pixel plane per 8-channel chunk of the (<= 16-channel) concat
+            const uint32_t plane = thin_plane_bytes(HP);
+            mbar_expect_tx(bar_hfull + 8 * hs, (uint32_t)(m_chunks * HP * 16));
+            for (int q = 0; q < m_chunks; ++q) {       // <= 2 planes: source 0, or sources 0 and 1 with one chunk each
+              const int sq = q < s_src[0].chunks ? 0 : 1, cq = q - (sq ? s_src[0].chunks : 0);
+              const int nm = s_src[sq].n_mod;
+              tma_load_4d(h_base + hs * halo_stage_bytes + q * plane, &maps.m[sq * nph + ph], bar_hfull + 8 * hs, cq * 8, tx * 8 + hox,
+                          ty * 16 * MT + hoy, nm ? (n % nm) : n);
+            }
+            continue;
           }
           const int nmod = s_src[si].n_mod;
           mbar_expect_tx(bar_hfull + 8 * hs, (uint32_t)(HP * 128));
@@ -904,8 +919,13 @@ __global__ void __launch_bounds__(HaloCfg<BN>::kThreads, HaloCfg<BN>::kMinCtas) 
   } else {
     // ------------------------------------------------------------------ MMA issuer
     constexpr uint32_t idesc = make_idesc_bf16(kBM, BN, 0, 0);
-    const uint32_t ahi = desc_hi((uint32_t)(Wh * 128)), bhi = desc_hi(1024);
-    const uint32_t a_mstep = (uint32_t)(16 * Wh * 128) >> 4;   // descriptor start-field step between stacked M tiles
+    // compact halo: SWIZZLE_NONE, SBO = one halo row; the second K half of an MMA is the next pixel (8 channels: x-adjacent tap,
+    // LBO = 16 B) or the next plane (16 channels); weights [K half][BN][16 B] (LBO = BN x 16 B, SBO = 128 B)
+    const uint32_t ahi = thin ? desc_hi_noswz((uint32_t)(Wh * 16)) : desc_hi((uint32_t)(Wh * 128));
+    const uint32_t bhi = thin ? desc_hi_noswz(128u) : desc_hi(1024);
+    const uint32_t a_lbo = thin ? (m_chunks == 1 ? 16u : thin_plane_bytes(HP)) : 16u, b_lbo = thin ? (uint32_t)(BN * 16) : 16u;
+    const uint32_t a_mstep = (uint32_t)(16 * Wh * (thin ? 16 : 128)) >> 4;   // descriptor start-field step between stacked M tiles
+    const uint32_t bstep = (uint32_t)kBStage >> 4;
     int bs = 0, hs = 0, it = 0;
     uint32_t bph = 0, hph = 0;
     int vlast = nchunks * nph - 1;                       // last virtual chunk that has taps
@@ -919,19 +939,19 @@ __global__ void __launch_bounds__(HaloCfg<BN>::kThreads, HaloCfg<BN>::kMinCtas) 
       const int nk16 = rem >= 8 ? 4 : (rem + 1) / 2;
       mbar_wait(bar_hfull + 8 * hs, hph);
       if (vc == 0 && lane == 0) CIS_TRACE_AT(1);
-      const uint32_t hlo = desc_lo(h_base + hs * halo_stage_bytes, 16);
+      const uint32_t hlo = desc_lo(h_base + hs * halo_stage_bytes, a_lbo);
       for (int t0 = tlo; t0 < thi; t0 += G, ++it) {
         const int gt = min(G, thi - t0);
         mbar_wait(bar_bfull + 8 * bs, bph);
         tc_fence_after();
         if (elect_one()) {
           CIS_TRACE_AT(8 + 2 * it);
-          const uint32_t blo = desc_lo(b_base + bs * stage_bytes, 16);
+          const uint32_t blo = desc_lo(b_base + bs * stage_bytes, b_lbo);
           const bool first = !any;
-          if (nk16 == 4) halo_issue_stage<4>(tmem, hlo, blo, s_aoff + t0, gt, MT, BN, ahi, bhi, a_mstep, idesc, first);
-          else if (nk16 == 1) halo_issue_stage<1>(tmem, hlo, blo, s_aoff + t0, gt, MT, BN, ahi, bhi, a_mstep, idesc, first);
-          else if (nk16 == 2) halo_issue_stage<2>(tmem, hlo, blo, s_aoff + t0, gt, MT, BN, ahi, bhi, a_mstep, idesc, first);
-          else halo_issue_stage<3>(tmem, hlo, blo, s_aoff + t0, gt, MT, BN, ahi, bhi, a_mstep, idesc, first);
+          if (nk16 == 4) halo_issue_stage<4>(tmem, hlo, blo, s_aoff + t0, gt, MT, BN, ahi, bhi, a_mstep, bstep, idesc, first);
+          else if (nk16 == 1) halo_issue_stage<1>(tmem, hlo, blo, s_aoff + t0, gt, MT, BN, ahi, bhi, a_mstep, bstep, idesc, first);
+          else if (nk16 == 2) halo_issue_stage<2>(tmem, hlo, blo, s_aoff + t0, gt, MT, BN, ahi, bhi, a_mstep, bstep, idesc, first);
+          else halo_issue_stage<3>(tmem, hlo, blo, s_aoff + t0, gt, MT, BN, ahi, bhi, a_mstep, bstep, idesc, first);
           umma_commit(bar_bempty + 8 * bs);
           if (t0 + G >= thi) {
             umma_commit(bar_hempty + 8 * hs);
@@ -1045,7 +1065,8 @@ template <int BN>
 __global__ void __launch_bounds__(kPThreads, 2) conv_halo_persist_kernel(const __grid_constant__ CisConv p, const int halo_stage_bytes,
                                                                        const int BS, const int NHS, const int AS, const int G,
                                                                        const __grid_constant__ HaloMaps maps, const int ws) {
-  constexpr int kBStage = BN * 128;
+  const int thin = p.thin;                       // compact thin halo: see conv_halo_kernel
+  const int kBStage = thin ? BN * 32 : BN * 128;
   constexpr int kMaxHS = 4;
   extern __shared__ uint8_t smem_raw[];
   __shared__ uint64_t bars[2 * kMaxHS + 2 * kHaloMaxBStages + 4];
@@ -1073,7 +1094,7 @@ __global__ void __launch_bounds__(kPThreads, 2) conv_halo_persist_kernel(const _
   const uint32_t ncols = want <= 32 ? 32u : want <= 64 ? 64u : want <= 128 ? 128u : want <= 256 ? 256u : 512u;
 
   pdl_launch_dependents();
-  if (tid < p.ntaps) s_aoff[tid] = (uint32_t)((p.dh[tid] * Wh + p.dw[tid]) * 8);
+  if (tid < p.ntaps) s_aoff[tid] = (uint32_t)((p.dh[tid] * Wh + p.dw[tid]) * (thin ? 1 : 8));
   if (warp == 3) {
     if (lane == 0) {
       for (int s = 0; s < NHS; ++s) {
@@ -1119,13 +1140,24 @@ __global__ void __launch_bounds__(kPThreads, 2) conv_halo_persist_kernel(const _
             c -= p.src[si].chunks;
             ++si;
           }
-          int nmod = p.src[0].n_mod;
-          if (si == 1) nmod = p.src[1].n_mod;
-          if (si == 2) nmod = p.src[2].n_mod;
-          if (si == 3) nmod = p.src[3].n_mod;
-          mbar_expect_tx(bar_hfull + 8 * hs, (uint32_t)(HP * 128));
-          tma_load_4d(h_base + hs * halo_stage_bytes, &maps.m[si], bar_hfull + 8 * hs, c * 8, tx * 8 + p.hox, ty * 16 * MT + p.hoy,
-                      nmod ? (n % nmod) : n);
+          if (thin) {
+            const uint32_t plane = thin_plane_bytes(HP);
+            mbar_expect_tx(bar_hfull + 8 * hs, (uint32_t)(m_chunks * HP * 16));
+            for (int q = 0; q < m_chunks; ++q) {       // <= 2 planes: source 0, or sources 0 and 1 with one chunk each
+              const int sq = q < p.src[0].chunks ? 0 : 1, cq = q - (sq ? p.src[0].chunks : 0);
+              const int nm = sq ? p.src[1].n_mod : p.src[0].n_mod;
+              tma_load_4d(h_base + hs * halo_stage_bytes + q * plane, &maps.m[sq], bar_hfull + 8 * hs, cq * 8, tx * 8 + p.hox,
+                          ty * 16 * MT + p.hoy, nm ? (n % nm) : n);
+            }
+          } else {
+            int nmod = p.src[0].n_mod;
+            if (si == 1) nmod = p.src[1].n_mod;
+            if (si == 2) nmod = p.src[2].n_mod;
+            if (si == 3) nmod = p.src[3].n_mod;
+            mbar_expect_tx(bar_hfull + 8 * hs, (uint32_t)(HP * 128));
+            tma_load_4d(h_base + hs * halo_stage_bytes, &maps.m[si], bar_hfull + 8 * hs, c * 8, tx * 8 + p.hox, ty * 16 * MT + p.hoy,
+                        nmod ? (n % nmod) : n);
+          }
           if (++hs == NHS) {
             hs = 0;
             hph ^= 1u;
@@ -1168,8 +1200,11 @@ __global__ void __launch_bounds__(kPThreads, 2) conv_halo_persist_kernel(const _
   } else if (warp == 2) {
     // ------------------------------------------------------------------ MMA issuer
     constexpr uint32_t idesc = make_idesc_bf16(kBM, BN, 0, 0);
-    const uint32_t ahi = desc_hi((uint32_t)(Wh * 128)), bhi = desc_hi(1024);
-    const uint32_t a_mstep = (uint32_t)(16 * Wh * 128) >> 4;
+    const uint32_t ahi = thin ? desc_hi_noswz((uint32_t)(Wh * 16)) : desc_hi((uint32_t)(Wh * 128));
+    const uint32_t bhi = thin ? desc_hi_noswz(128u) : desc_hi(1024);
+    const uint32_t a_lbo = thin ? (m_chunks == 1 ? 16u : thin_plane_bytes(HP)) : 16u, b_lbo = thin ? (uint32_t)(BN * 16) : 16u;
+    const uint32_t a_mstep = (uint32_t)(16 * Wh * (thin ? 16 : 128)) >> 4;
+    const uint32_t bstep = (uint32_t)kBStage >> 4;
     int hs = 0, bs = 0, as = 0;
     uint32_t hph = 0, bph = 0, tph = 1;
     if (ws && (int)blockIdx.x < total) {
@@ -1188,19 +1223,19 @@ __global__ void __launch_bounds__(kPThreads, 2) conv_halo_persist_kernel(const _
         const int nk16 = rem >= 8 ? 4 : (rem + 1) / 2;
         mbar_wait(bar_hfull + 8 * hs, hph);
         if (cc == 0 && lane == 0) CIS_TRACE_AT(10 + 5 * wi);
-        const uint32_t hlo = desc_lo(h_base + hs * halo_stage_bytes, 16);
+        const uint32_t hlo = desc_lo(h_base + hs * halo_stage_bytes, a_lbo);
         const int gstep = ws ? p.ntaps : G;
         for (int t0 = 0; t0 < p.ntaps; t0 += gstep) {
           const int gt = min(gstep, p.ntaps - t0);
           if (!ws) mbar_wait(bar_bfull + 8 * bs, bph);
           tc_fence_after();
           if (elect_one()) {
-            const uint32_t blo = desc_lo(ws ? b_base + (uint32_t)(cc * p.ntaps) * kBStage : b_base + bs * stage_bytes, 16);
+            const uint32_t blo = desc_lo(ws ? b_base + (uint32_t)(cc * p.ntaps) * kBStage : b_base + bs * stage_bytes, b_lbo);
             const bool first = (cc | t0) == 0;
-            if (nk16 == 4) halo_issue_stage<4>(tacc, hlo, blo, s_aoff + t0, gt, MT, BN, ahi, bhi, a_mstep, idesc, first);
-            else if (nk16 == 1) halo_issue_stage<1>(tacc, hlo, blo, s_aoff + t0, gt, MT, BN, ahi, bhi, a_mstep, idesc, first);
-            else if (nk16 == 2) halo_issue_stage<2>(tacc, hlo, blo, s_aoff + t0, gt, MT, BN, ahi, bhi, a_mstep, idesc, first);
-            else halo_issue_stage<3>(tacc, hlo, blo, s_aoff + t0, gt, MT, BN, ahi, bhi, a_mstep, idesc, first);
+            if (nk16 == 4) halo_issue_stage<4>(tacc, hlo, blo, s_aoff + t0, gt, MT, BN, ahi, bhi, a_mstep, bstep, idesc, first);
+            else if (nk16 == 1) halo_issue_stage<1>(tacc, hlo, blo, s_aoff + t0, gt, MT, BN, ahi, bhi, a_mstep, bstep, idesc, first);
+            else if (nk16 == 2) halo_issue_stage<2>(tacc, hlo, blo, s_aoff + t0, gt, MT, BN, ahi, bhi, a_mstep, bstep, idesc, first);
+            else halo_issue_stage<3>(tacc, hlo, blo, s_aoff + t0, gt, MT, BN, ahi, bhi, a_mstep, bstep, idesc, first);
             if (!ws) umma_commit(bar_bempty + 8 * bs);
             if (t0 + gstep >= p.ntaps) {
               umma_commit(bar_hempty + 8 * hs);
@@ -1734,8 +1769,9 @@ static EncodeTiledFn get_encode_tiled() {
 // space-to-depth phase (py, px) of the image: pixel (y, x) of the map is input pixel (2y + py, 2x + px).
 // step/py/px: a stride-2 phase view (coarser grid through the global strides, phase offset in the base address).
 // estride: dilated layers -- ONE map per source, every estride-th pixel of a box that starts at any (phase-carrying) coordinate.
+// thin: compact thin halo -- box (8, bw, bh, 1) without swizzle, one 16-byte-per-pixel plane per load (CisConv.thin).
 static bool encode_src_map(CUtensorMap* m, const CisSrc& s, int N, int H, int W, int bw, int bh, int step = 1, int py = 0, int px = 0,
-                           int estride = 1) {
+                           int estride = 1, bool thin = false) {
   EncodeTiledFn enc = get_encode_tiled();
   if (!enc) return false;
   const int nb = s.n_mod > 0 ? s.n_mod : N;
@@ -1743,10 +1779,11 @@ static bool encode_src_map(CUtensorMap* m, const CisSrc& s, int N, int H, int W,
   if (Hq < 1 || Wq < 1) return false;
   cuuint64_t dims[4] = {(cuuint64_t)s.chunks * 8, (cuuint64_t)Wq, (cuuint64_t)Hq, (cuuint64_t)nb};
   cuuint64_t strides[3] = {(cuuint64_t)step * s.pitch * 2, (cuuint64_t)step * W * s.pitch * 2, (cuuint64_t)H * W * s.pitch * 2};
-  cuuint32_t box[4] = {64, (cuuint32_t)(bw * estride), (cuuint32_t)(bh * estride), 1};   // extent in the un-strided pixel space
+  cuuint32_t box[4] = {thin ? 8u : 64u, (cuuint32_t)(bw * estride), (cuuint32_t)(bh * estride), 1};   // extent in the un-strided pixel space
   cuuint32_t es[4] = {1, (cuuint32_t)estride, (cuuint32_t)estride, 1};
   void* base = (void*)((const char*)s.ptr + ((size_t)(py * W + px) * s.pitch + (size_t)s.c_off) * 2);
-  return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, base, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
+  return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, base, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
+             thin ? CU_TENSOR_MAP_SWIZZLE_NONE : CU_TENSOR_MAP_SWIZZLE_128B,
              CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
@@ -1767,14 +1804,17 @@ extern "C" int cis_set_persist_mode(int mode) {
 template <int BN>
 static int launch_halo(const CisConv* d, cudaStream_t st) {
   const int Wh = 8 + d->ex, Hh = 16 * d->MT + d->ey, HP = Wh * Hh;
-  const int halo_stage = (HP * 128 + 1023) & ~1023;
   int chunks = 0;
   for (int i = 0; i < d->nsrc; ++i) chunks += d->src[i].chunks;
+  const bool thin = d->thin != 0;
+  if (thin && (chunks > 2 || d->dil != 1 || d->splits > 1))
+    return cis_set_error(CIS_ERR_BAD_ARG, "cis_conv_igemm(halo): the compact thin halo takes <= 16 channels, no dilation, no split-K");
+  const int halo_stage = thin ? (int)((chunks * thin_plane_bytes(HP) + 1023) & ~1023u) : (HP * 128 + 1023) & ~1023;
   const int nchunks = (chunks + 7) / 8;
   const int nsub = d->nsub > 1 ? d->nsub : 1;                  // grouped launch: grid.z = sub-problem, no split-K
   const int nsp = (nsub == 1 && d->splits > 1) ? d->splits : 1;
   const int cper = (nchunks + nsp - 1) / nsp;                  // 64-channel chunks per CTA
-  const int nhs = cper > 1 ? 2 : 1;                            // halo stages: double-buffer only when there is a next chunk to prefetch
+  const int nhs = cper * (d->nph > 1 ? d->nph : 1) > 1 ? 2 : 1; // halo stages: double-buffer only when there is a next chunk / phase to prefetch
   const int dd = d->dil;
   int tiles = 0, ntaps_max = d->ntaps;
   if (nsub > 1) {
@@ -1797,7 +1837,7 @@ static int launch_halo(const CisConv* d, cudaStream_t st) {
   // ---- weight pipeline: G taps per stage (one bulk copy, one wait / commit of the MMA thread), BS stages
   static const int g_env = getenv("CIS_HALO_G") ? atoi(getenv("CIS_HALO_G")) : 0;            // experiments: force the group size
   static const int stage_kb = getenv("CIS_HALO_STAGE_KB") ? atoi(getenv("CIS_HALO_STAGE_KB")) : 48;
-  const int kB = BN * 128;
+  const int kB = thin ? BN * 32 : BN * 128;     // weight bytes per tap (compact: per K=16 MMA)
   int G = g_env > 0 ? g_env : (stage_kb * 1024) / kB;
   if (G < 1) G = 1;
   if (G > ntaps_max) G = ntaps_max;
@@ -1837,14 +1877,15 @@ static int launch_halo(const CisConv* d, cudaStream_t st) {
   const int nph = d->nph > 1 ? d->nph : 1;
   static const int dil_tma = getenv("CIS_DIL_TMA") ? atoi(getenv("CIS_DIL_TMA")) : 1;
   int use_tma = ((d->dil == 1 || dil_tma) && Wh * d->dil <= 256 && Hh * d->dil <= 256) ? 1 : 0;
-  for (int i = 0; use_tma && i < d->nsrc - 1; ++i)
+  for (int i = 0; use_tma && !thin && i < d->nsrc - 1; ++i)     // (compact planes are 8 channels: they never straddle sources)
     if (d->src[i].chunks % 8) use_tma = 0;
   for (int i = 0; use_tma && i < d->nsrc; ++i) {
     if (((uintptr_t)d->src[i].ptr + (size_t)d->src[i].c_off * 2) % 16) use_tma = 0;
     for (int ph = 0; use_tma && ph < nph; ++ph)
-      if (!encode_src_map(&maps.m[i * nph + ph], d->src[i], d->N, d->H, d->W, Wh, Hh, nph > 1 ? 2 : 1, ph >> 1, ph & 1, d->dil)) use_tma = 0;
+      if (!encode_src_map(&maps.m[i * nph + ph], d->src[i], d->N, d->H, d->W, Wh, Hh, nph > 1 ? 2 : 1, ph >> 1, ph & 1, d->dil, thin)) use_tma = 0;
   }
   if (!use_tma) memset(&maps, 0, sizeof(maps));
+  if (thin && !use_tma) return cis_set_error(CIS_ERR_UNSUPPORTED, "cis_conv_igemm(halo): the compact thin halo needs the TMA halo path");
   if (nph > 1 && !use_tma) return cis_set_error(CIS_ERR_UNSUPPORTED, "cis_conv_igemm(halo): stride-2 phases need the TMA halo path");
   // persistent variant (conv_halo_persist_kernel): layers with many tiles per SM.  CIS_PERSIST_MODE / cis_set_persist_mode:
   //   0 off | 1 (default) layers whose whole weight set stays resident in shared memory and that have >= 2 tiles per SM |

@@ -43,19 +43,30 @@ __device__ __forceinline__ void pack_weights_body(size_t i, const float* __restr
 }
 // Pre-swizzled weight tiles for the halo kernel: block (ny, cc, t) = BN rows x 128 B, row n holds K = 64 channels of chunk cc for
 // tap t with the SWIZZLE_128B pattern already applied (16-byte chunk index ^= n & 7), so a plain bulk copy lands the UMMA layout.
+// layout 1 (compact thin halo, CisConv.thin): cin8 = 16 K positions per "tap" (= one K=16 MMA), block t = BN x 32 B in the no-swizzle
+// K-major canonical layout [K half][n][8]: core matrices of 8 n-rows x 16 B, 128 B apart along n (SBO), BN x 16 B apart along K (LBO).
+__device__ __forceinline__ int tiled_kk(int q, int BN, int layout, int& n) {
+  if (layout) {
+    n = (q >> 3) % BN;
+    return ((q / (BN * 8)) << 3) | (q & 7);
+  }
+  n = q >> 6;
+  const int pos = q & 63;                    // physical element position inside the 128-byte row
+  return (((pos >> 3) ^ (n & 7)) << 3) | (pos & 7);   // logical channel within the chunk
+}
 __device__ __forceinline__ void pack_weights_tiled_body(size_t i, const float* __restrict__ w, const int* __restrict__ kmap, int cin8, int ntaps,
                                                         int n_tiles, int BN, int cout, int sn, const int* __restrict__ nmap,
-                                                        bf16* __restrict__ out) {
+                                                        bf16* __restrict__ out, int layout) {
   const int nchunks = (cin8 + 63) / 64;
-  const size_t total = (size_t)n_tiles * nchunks * ntaps * BN * 64;
+  const int KT = layout ? 16 : 64;
+  const size_t total = (size_t)n_tiles * nchunks * ntaps * BN * KT;
   if (i >= total) return;
-  const int pos = (int)(i % 64);            // physical element position inside the 128-byte row
-  size_t r = i / 64;
-  const int n = (int)(r % BN); r /= BN;
+  size_t r = i / ((size_t)BN * KT);
+  int n;
+  const int kk = tiled_kk((int)(i % ((size_t)BN * KT)), BN, layout, n);
   const int t = (int)(r % ntaps); r /= ntaps;
   const int cc = (int)(r % nchunks);
   const int ny = (int)(r / nchunks);
-  const int kk = (((pos >> 3) ^ (n & 7)) << 3) | (pos & 7);   // logical channel within the chunk
   const int c = cc * 64 + kk;
   float v = 0.f;
   if (c < cin8) {
@@ -71,13 +82,14 @@ __device__ __forceinline__ void pack_weights_tiled_body(size_t i, const float* _
 // form above reads a column of the [tap*cin][cout] matrix per warp: 4 useful bytes per 32-byte sector.  tile: >= 64 * (BN + 1) floats.
 __device__ __forceinline__ void pack_weights_tiled_tile(int blk, const float* __restrict__ w, const int* __restrict__ kmap, int cin8, int ntaps,
                                                         int n_tiles, int BN, int cout, const int* __restrict__ nmap, bf16* __restrict__ out,
-                                                        float* tile) {
+                                                        float* tile, int layout) {
   const int nchunks = (cin8 + 63) / 64;
+  const int KT = layout ? 16 : 64;
   const int t = blk % ntaps;
   const int r = blk / ntaps;
   const int cc = r % nchunks, ny = r / nchunks;
   const int ld = BN + 1;
-  for (int idx = threadIdx.x; idx < BN * 64; idx += blockDim.x) {
+  for (int idx = threadIdx.x; idx < BN * KT; idx += blockDim.x) {
     const int n = idx % BN, kk = idx / BN;
     const int c = cc * 64 + kk;
     float v = 0.f;
@@ -90,10 +102,10 @@ __device__ __forceinline__ void pack_weights_tiled_tile(int blk, const float* __
     tile[kk * ld + n] = v;
   }
   __syncthreads();
-  bf16* o = out + (size_t)blk * BN * 64;
-  for (int idx = threadIdx.x; idx < BN * 64; idx += blockDim.x) {
-    const int pos = idx & 63, n = idx >> 6;
-    const int kk = (((pos >> 3) ^ (n & 7)) << 3) | (pos & 7);
+  bf16* o = out + (size_t)blk * BN * KT;
+  for (int idx = threadIdx.x; idx < BN * KT; idx += blockDim.x) {
+    int n;
+    const int kk = tiled_kk(idx, BN, layout, n);
     o[idx] = __float2bfloat16(tile[kk * ld + n]);
   }
 }
@@ -179,12 +191,12 @@ __global__ void pack_weights_kernel(const float* __restrict__ w, const int* __re
   pack_weights_body((size_t)blockIdx.x * blockDim.x + threadIdx.x, w, kmap, K_pad, rows, cout, sn, nmap, wp);
 }
 __global__ void pack_weights_tiled_kernel(const float* __restrict__ w, const int* __restrict__ kmap, int cin8, int ntaps, int n_tiles, int BN,
-                                          int cout, int sn, const int* __restrict__ nmap, bf16* __restrict__ out) {
+                                          int cout, int sn, const int* __restrict__ nmap, bf16* __restrict__ out, int layout) {
   pdl_launch_dependents();
   pdl_wait();
   __shared__ float tile[64 * 129];
-  if (sn == 1) pack_weights_tiled_tile(blockIdx.x, w, kmap, cin8, ntaps, n_tiles, BN, cout, nmap, out, tile);
-  else pack_weights_tiled_body((size_t)blockIdx.x * blockDim.x + threadIdx.x, w, kmap, cin8, ntaps, n_tiles, BN, cout, sn, nmap, out);
+  if (sn == 1) pack_weights_tiled_tile(blockIdx.x, w, kmap, cin8, ntaps, n_tiles, BN, cout, nmap, out, tile, layout);
+  else pack_weights_tiled_body((size_t)blockIdx.x * blockDim.x + threadIdx.x, w, kmap, cin8, ntaps, n_tiles, BN, cout, sn, nmap, out, layout);
 }
 __global__ void unpack_wgrad_kernel(const float* __restrict__ dwp, const int* __restrict__ kmap, int K_pad, int cout, int nsplit,
                                     float* __restrict__ dw, const float* __restrict__ colpart, int nblocks, int nch, float* __restrict__ db,
@@ -229,10 +241,10 @@ __global__ void param_multi_kernel(const CisParamJob* __restrict__ jobs, int njo
     case CIS_JOB_PACK_TILED:
       if (j.i[5] == 1)       // forward orientation: one block per tile, transposed through shared memory
         pack_weights_tiled_tile(blk, (const float*)j.p[0], (const int*)j.p[1], j.i[0], j.i[1], j.i[2], j.i[3], j.i[4], (const int*)j.p[2],
-                                (bf16*)j.p[3], tile);
+                                (bf16*)j.p[3], tile, j.i[6]);
       else
         pack_weights_tiled_body(i, (const float*)j.p[0], (const int*)j.p[1], j.i[0], j.i[1], j.i[2], j.i[3], j.i[4], j.i[5], (const int*)j.p[2],
-                                (bf16*)j.p[3]);
+                                (bf16*)j.p[3], j.i[6]);
       break;
     case CIS_JOB_UNPACK:
       unpack_wgrad_body(i, (const float*)j.p[0], (const int*)j.p[1], j.i[0], j.i[1], j.i[2], (float*)j.p[2], (const float*)j.p[3], j.i[3], j.i[4],
@@ -1214,11 +1226,12 @@ int cis_pack_weights(const float* w, const int32_t* kmap, int32_t K_pad, int32_t
   return cis_check_launch("pack_weights");
 }
 int cis_pack_weights_tiled(const float* w, const int32_t* kmap, int32_t cin8, int32_t ntaps, int32_t n_tiles, int32_t BN, int32_t cout, int32_t sn,
-                           const int32_t* nmap, void* out, cis_stream_t stream) {
+                           const int32_t* nmap, void* out, int32_t layout, cis_stream_t stream) {
+  if (layout && cin8 != 16) return cis_set_error(CIS_ERR_BAD_ARG, "cis_pack_weights_tiled: layout 1 packs 16 K positions per tile");
   const size_t total = (size_t)n_tiles * ((cin8 + 63) / 64) * ntaps * BN * 64;
   const unsigned blocks = sn == 1 ? (unsigned)(n_tiles * ((cin8 + 63) / 64) * ntaps) : nblk(total);
   if (BN > 128) return cis_set_error(CIS_ERR_UNSUPPORTED, "cis_pack_weights_tiled: BN > 128");
-  CIS_LAUNCH(pack_weights_tiled_kernel, blocks, 256, 0, ST, w, kmap, cin8, ntaps, n_tiles, BN, cout, sn, nmap, (mbf)out);
+  CIS_LAUNCH(pack_weights_tiled_kernel, blocks, 256, 0, ST, w, kmap, cin8, ntaps, n_tiles, BN, cout, sn, nmap, (mbf)out, layout);
   return cis_check_launch("pack_weights_tiled");
 }
 int cis_unpack_wgrad(const float* dwp, const int32_t* kmap, int32_t K_pad, int32_t cout, int32_t nsplit, float* dw, const float* colpart,

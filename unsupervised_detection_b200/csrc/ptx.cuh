@@ -195,6 +195,8 @@ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr, uint32_t lbo_
 }
 // Split form for hot issue loops: hi word is loop-invariant, lo word = start>>4 | LBO>>4<<16 advances by (bytes>>4) per K step.
 __device__ __forceinline__ uint32_t desc_hi(uint32_t sbo_bytes) { return ((sbo_bytes >> 4) & 0x3FFF) | (1u << 14) | (2u << 29); }
+// hi word of a SWIZZLE_NONE descriptor (layout 0): K-major core matrices of 8 rows x 16 B, LBO = K-direction step, SBO = 8-row step
+__device__ __forceinline__ uint32_t desc_hi_noswz(uint32_t sbo_bytes) { return ((sbo_bytes >> 4) & 0x3FFF) | (1u << 14); }
 __device__ __forceinline__ uint32_t desc_lo(uint32_t saddr, uint32_t lbo_bytes) {
   return ((saddr & 0x3FFFF) >> 4) | (((lbo_bytes >> 4) & 0x3FFF) << 16);
 }
